@@ -4,6 +4,7 @@ TwoTower-style retrieval, 10 M users x 1 M items, embed 64, top-100, consumed fi
 
     python bench.py --gpus 1 --steps 20 --warmup 3            # this repo's CUDA path
     python bench.py --impl reference --steps 3 --warmup 1     # reference algorithm on host cores
+    python bench.py --steps 5 --dump-outputs DIR              # + the last timed step's ids as DIR/*.npy
     torchrun --nproc-per-node N ... bench.py --gpus N ...     # one rank per GPU (users sharded)
 
 One JSON line on rank 0 (see the driver contract).  A "step" = one recommend call for a batch of
@@ -53,7 +54,15 @@ def parse():
                          "configurations on one GPU (librecommender_b200/bench_configs.py)")
     ap.add_argument("--epi-warps", type=int, default=0, help="tuning: epilogue warps per TMEM quadrant (2|3)")
     ap.add_argument("--pre-coef", type=float, default=0.0, help="tuning: speculative rank coefficient")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the results of the last timed step of rank 0 (device leg "
+                         "and end-to-end leg) as DIR/<name>.npy in float64, to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.config != "c2"):
+        ap.error("--dump-outputs writes the results of the CUDA path of --config c2 (--impl b200)")
+    return args
 
 
 # --------------------------------------------------------------------------------------------
@@ -116,6 +125,25 @@ def make_consumed_csr(args, device):
 def make_batches(args, rank, n):
     rng = np.random.default_rng(SEED_Q + 1000 * rank)
     return [rng.choice(args.users, size=args.batch, replace=False).astype(np.int64) for _ in range(n)]
+
+
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(dirname, arrays):
+    """Write each [B, ...] result as <dirname>/<name>.npy in float64 (item ids are exact there).  Above
+    DUMP_BYTES in all, every array keeps the same fixed, seeded sample of rows (rows.npy lists them)."""
+    host = {k: np.asarray(v.cpu().numpy() if hasattr(v, "cpu") else v, dtype=np.float64) for k, v in arrays.items()}
+    if sum(a.nbytes for a in host.values()) > DUMP_BYTES:
+        n = next(iter(host.values())).shape[0]
+        row_bytes = sum(a[0].nbytes for a in host.values()) + 8          # + its entry in rows.npy
+        keep = (DUMP_BYTES - 4096) // row_bytes                          # 4096: room for the .npy headers
+        rows = np.sort(np.random.default_rng(SEED_Q + 2000).choice(n, keep, replace=False))
+        host = {k: a[rows] for k, a in host.items()}
+        host["rows"] = rows.astype(np.float64)
+    os.makedirs(dirname, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(dirname, f"{k}.npy"), a)
 
 
 # --------------------------------------------------------------------------------------------
@@ -408,6 +436,8 @@ def main():
     e2e_ms = max_over_ranks(e0.elapsed_time(e1))
     e2e_value = world * args.batch * args.steps / (e2e_ms * 1e-3)
     assert res.shape == (args.batch, args.topk) and res.dtype == np.int64 and (res >= 0).all()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"device_ids": out, "e2e_ids": res})
 
     # ---- parity of one TIMED batch, outside the timed region: fused result vs the exact path ----
     last = batches_d[n_batches - 1]

@@ -1,12 +1,19 @@
 """Host logic of the recommendation shims: id re-mapping (construct_rec) and argument validation
-(check_dynamic_rec_feats) — compared with the unmodified reference when it is importable
-(libreco/recommendation/recommend.py:8-18,39-54)."""
+(check_dynamic_rec_feats) and cold-start draws — compared with the answers of the unmodified reference
+(libreco/recommendation/recommend.py:8-18,39-54, cold_start.py) stored in tests/golden/reference_answers.npz
+(tests/golden/gen_reference_answers.py)."""
 import types
 
 import numpy as np
 import pytest
 
-from oracle.ref_loader import load_reference, reference_available
+from _fixtures import load_reference_answers
+
+CONSTRUCT_USERS = [1, 2, 5, 4]
+CHECK_ARGS = (("DeepFM", 1, None, [1]), ("DIN", [1, 2], {"a": 1}, None), ("DIN", 1, None, (1,)),
+              ("DIN", 1, [1], None), ("YouTubeRanking", 1, None, [3, 4]))
+COLD_USERS = ["u9", "u3", "u5"]
+COLD_DEFAULT_RECS = np.arange(5, 25)
 
 
 def _data_info(n_users=7, n_items=50, str_items=False):
@@ -40,21 +47,20 @@ def test_construct_rec_maps_inner_to_original(str_items):
     assert out2[di2.id2user[3]].tolist() == [di2.id2item[i] for i in recs[0]]
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference not mounted")
-def test_construct_rec_equals_reference():
-    load_reference()
-    from libreco.recommendation.recommend import construct_rec as ref_construct
+def construct_recs():
+    return np.random.default_rng(2).integers(0, 50, size=(4, 12))
 
+
+def test_construct_rec_equals_reference():
     from librecommender_b200.recommendation import construct_rec
 
+    g = load_reference_answers()
     di = _data_info()
-    recs = np.random.default_rng(2).integers(0, 50, size=(4, 12))
     for inner in (True, False):
-        a = construct_rec(di, [1, 2, 5, 4], recs, inner)
-        b = ref_construct(di, [1, 2, 5, 4], recs, inner)
-        assert list(a) == list(b)
-        for k in a:
-            np.testing.assert_array_equal(a[k], b[k])
+        a = construct_rec(di, CONSTRUCT_USERS, construct_recs(), inner)
+        assert list(a) == g[f"construct_{inner}_keys"].tolist()
+        for k, want in zip(a, g[f"construct_{inner}_vals"]):
+            np.testing.assert_array_equal(a[k], want)
 
 
 def test_check_dynamic_rec_feats_errors():
@@ -71,23 +77,14 @@ def test_check_dynamic_rec_feats_errors():
         check_dynamic_rec_feats("DIN", 1, None, (1, 2))
     with pytest.raises(ValueError, match="must be `dict`"):
         check_dynamic_rec_feats("DIN", 1, [("sex", "F")], None)
-    if reference_available():
-        load_reference()
-        from libreco.recommendation.recommend import check_dynamic_rec_feats as ref_check
-
-        for args in (("DeepFM", 1, None, [1]), ("DIN", [1, 2], {"a": 1}, None), ("DIN", 1, None, (1,)),
-                     ("DIN", 1, [1], None), ("YouTubeRanking", 1, None, [3, 4])):
-            try:
-                ref_check(*args)
-                ref_err = None
-            except ValueError as e:
-                ref_err = str(e)
-            try:
-                check_dynamic_rec_feats(*args)
-                our_err = None
-            except ValueError as e:
-                our_err = str(e)
-            assert ref_err == our_err
+    # the reference's messages for the same arguments ("" where it accepts them)
+    for args, ref_err in zip(CHECK_ARGS, load_reference_answers()["check_messages"].tolist(), strict=True):
+        try:
+            check_dynamic_rec_feats(*args)
+            our_err = ""
+        except ValueError as e:
+            our_err = str(e)
+        assert ref_err == our_err
 
 
 def test_recommend_tf_feat_requires_engine_and_validates():
@@ -118,8 +115,8 @@ def test_cold_start_rec_draws_like_the_reference(strategy, inner_id):
     """cold_start.py: one np_rng.choice(pool, n_rec) per user, in user order, with replacement."""
     from librecommender_b200.recommendation import cold_start_rec
 
-    default_recs = np.arange(5, 25)
-    users = ["u9", "u3", "u5"]
+    default_recs = COLD_DEFAULT_RECS
+    users = COLD_USERS
     got = cold_start_rec(_cold_data_info(), default_recs, strategy, users, 6, inner_id)
     di = _cold_data_info()
     assert list(got) == users
@@ -131,12 +128,7 @@ def test_cold_start_rec_draws_like_the_reference(strategy, inner_id):
             picked = di.np_rng.choice(di.popular_items, 6)
             want = np.array([di.item2id[i] for i in picked]) if inner_id else picked
         np.testing.assert_array_equal(got[u], want)
-    if reference_available():
-        load_reference()
-        from libreco.recommendation.cold_start import cold_start_rec as ref_cold
-
-        ref = ref_cold(_cold_data_info(), default_recs, strategy, users, 6, inner_id)
-        for u in users:
-            np.testing.assert_array_equal(got[u], ref[u])
+    for u, want in zip(users, load_reference_answers()[f"cold_{strategy}_{inner_id}"]):
+        np.testing.assert_array_equal(got[u], want)
     with pytest.raises(ValueError, match="Unknown cold start strategy"):
         cold_start_rec(_cold_data_info(), default_recs, "nearest", users, 6, inner_id)

@@ -1,70 +1,64 @@
-"""Host-side inference plumbing against the UNMODIFIED reference (mounted /root/reference or the staged
-oracle/_ref): per-row features of "one user x every item" with user features overridden
-(recommendation/preprocess.py:104-212 + prediction/preprocess.py:58-104), the padded sequence row
-(recommendation/preprocess.py:36-45) and the OOV-row assignment rule (bases/tf_base.py:310-353, restated
-because it is a TensorFlow graph op)."""
-import types
-
+"""Host-side inference plumbing against the UNMODIFIED reference, whose answers on the C1 DataInfo
+(DatasetFeat on sample_movielens_merged.csv) are stored in tests/golden/reference_answers.npz
+(tests/golden/gen_reference_answers.py): per-row features of "one user x every item" with user features
+overridden (recommendation/preprocess.py:104-212 + prediction/preprocess.py:58-104), the padded sequence
+row (recommendation/preprocess.py:36-45) and the OOV-row assignment rule (bases/tf_base.py:310-353,
+restated because it is a TensorFlow graph op)."""
 import numpy as np
 import pytest
 
-from oracle.ref_loader import REFERENCE_ROOT, load_reference, reference_available
+from _fixtures import load_feat_data_info, load_reference_answers
 
-pytestmark = pytest.mark.skipif(not reference_available(), reason="reference neither mounted nor staged")
+FEATS = [None, {"sex": "F", "age": 33.0}, {"occupation": 17, "nonexistent": 1},
+         {"sex": "no-such-value", "age": 5.0, "genre1": "Comedy"}]
+
+
+def users(n_users):
+    return (0, 7, n_users)                                      # incl. the OOV user row
+
+
+def rec_seq_cases(id2item):
+    some = [id2item[i] for i in range(25)]
+    return ((list(range(3)), True), (list(range(40)), True), (some, False), (some[:4] + ["unknown"], False))
 
 
 @pytest.fixture(scope="module")
 def data_info():
-    import os
-
-    import pandas as pd
-
-    load_reference()
-    from libreco.data import DatasetFeat, split_by_ratio_chrono
-
-    path = os.path.join(REFERENCE_ROOT, "examples/sample_data/sample_movielens_merged.csv")
-    if not os.path.exists(path):
-        pytest.skip("sample_movielens_merged.csv not available (staged tree carries the rating file only)")
-    data = pd.read_csv(path)
-    train, _ = split_by_ratio_chrono(data, test_size=0.2)
-    _, di = DatasetFeat.build_trainset(train, ["sex", "age", "occupation"], ["genre1", "genre2", "genre3"],
-                                       ["sex", "occupation", "genre1", "genre2", "genre3"], ["age"])
-    return di
+    return load_feat_data_info()
 
 
-@pytest.mark.parametrize("feats", [None, {"sex": "F", "age": 33.0}, {"occupation": 17, "nonexistent": 1},
-                                   {"sex": "no-such-value", "age": 5.0, "genre1": "Comedy"}])
-def test_dynamic_feature_rows_equal_reference(data_info, feats):
-    from libreco.prediction.preprocess import set_temp_feats
-    from libreco.recommendation.preprocess import _get_original_feats
+@pytest.fixture(scope="module")
+def golden():
+    return load_reference_answers()
 
+
+@pytest.mark.parametrize("feats", FEATS)
+def test_dynamic_feature_rows_equal_reference(data_info, golden, feats):
     from librecommender_b200.dynamic_feats import dynamic_feature_rows
 
-    for user in (0, 7, data_info.n_users):                      # incl. the OOV user row
-        sp_ref, de_ref = _get_original_feats(data_info, user, data_info.n_items, True, True)
-        if feats is not None:
-            sp_ref, de_ref = set_temp_feats(data_info, sp_ref, de_ref, feats)
+    f = FEATS.index(feats)
+    assert golden["dyn_feats"][f] == repr(feats)
+    rows = golden["dyn_rows"]                                   # a fixed sample of the N item rows
+    for j, user in enumerate(users(data_info.n_users)):
+        case = f * 3 + j
         before = (data_info.user_sparse_unique.copy(), data_info.user_dense_unique.copy())
         sp, de = dynamic_feature_rows(data_info, user, feats)
-        np.testing.assert_array_equal(sp, sp_ref)
-        np.testing.assert_array_equal(de, de_ref)
+        assert sp.shape[0] == de.shape[0] == data_info.n_items
+        np.testing.assert_array_equal(sp[rows], golden["dyn_sparse"][case])
+        np.testing.assert_array_equal(de[rows], golden["dyn_dense"][case])
         np.testing.assert_array_equal(data_info.user_sparse_unique, before[0])      # nothing was modified
         np.testing.assert_array_equal(data_info.user_dense_unique, before[1])
 
 
-def test_build_rec_seq_equals_reference(data_info):
-    from libreco.recommendation.preprocess import build_rec_seq as ref_fn
-
+def test_build_rec_seq_equals_reference(data_info, golden):
     from librecommender_b200.dynamic_feats import build_rec_seq
 
-    model = types.SimpleNamespace(data_info=data_info, n_items=data_info.n_items, max_seq_len=10)
-    some = [data_info.id2item[i] for i in range(25)]
-    for seq, inner in ((list(range(3)), True), (list(range(40)), True), (some, False), (some[:4] + ["unknown"], False)):
-        ref_seq, ref_len = ref_fn(seq, model, inner)
+    for c, (seq, inner) in enumerate(rec_seq_cases(data_info.id2item)):
+        ref_seq, ref_len = golden["rec_seq"][c], golden["rec_seq_len"][c]
         got_seq, got_len = build_rec_seq(seq, data_info.n_items, 10, data_info.item2id, inner)
         np.testing.assert_array_equal(got_seq, ref_seq)
         np.testing.assert_array_equal(got_len, ref_len)
-        assert got_seq.dtype == ref_seq.dtype and got_len.dtype == ref_len.dtype
+        assert [str(got_seq.dtype), str(got_len.dtype)] == golden["rec_seq_dtypes"].tolist()
 
 
 def test_assign_oov_rows_rule(data_info):

@@ -8,6 +8,7 @@ vectors at several magnitudes, adversarial vectors whose every component sits at
 position, vectors with a huge dynamic range (fp16 subnormals — rounded AND flushed to zero), widths
 up to the kernel's limit, and a pessimistic model of the accumulator (truncation after every one of
 the d products)."""
+import os
 import re
 
 import numpy as np
@@ -15,7 +16,8 @@ import pytest
 
 
 def _src():
-    return open("librecommender_b200/csrc/score_topk_tc.cu").read()
+    return open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "librecommender_b200", "csrc",
+                     "score_topk_tc.cu")).read()
 
 
 def _err_coef():

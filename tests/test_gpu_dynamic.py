@@ -1,6 +1,6 @@
 """GPU: the a3 / a15 gaps closed in round 2, on the reference's own C1 data pipeline (DatasetFeat on
-sample_movielens_merged.csv, examples/feat_ranking_example.py:27-41; reference from /root/reference or
-the staged oracle/_ref):
+sample_movielens_merged.csv, examples/feat_ranking_example.py:27-41; its DataInfo and the reference's
+feeds are stored in tests/golden/movielens_feat.npz and tests/golden/reference_answers.npz):
 
 * single-user ``recommend_tf_feat`` with ``user_feats`` / ``seq`` supplied for the call
   (recommendation/recommend.py:39-54,81-105) == the numpy restatement of the model graph evaluated on
@@ -8,30 +8,23 @@ the staged oracle/_ref):
 * ``assign_oov`` on the device tables == the restated ``assign_tf_variables_oov`` rule, and
   ``default_recs`` == top-2000 of the OOV user without the consumed filter (bases/tf_base.py:145-153).
 The TF graph math itself stays parity-unpinned (no TensorFlow anywhere); the FEED is the reference's."""
-import os
 import types
 
 import numpy as np
 import pytest
 
-from oracle.ref_loader import REFERENCE_ROOT, load_reference, reference_available
+from _fixtures import load_feat_data_info, load_reference_answers
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not reference_available(), reason="reference neither mounted nor staged")]
+pytestmark = pytest.mark.gpu
+
+
+def override_cases(n_users):
+    return ((5, {"sex": "F", "age": 40.0}), (11, {"occupation": 3}), (n_users, {"age": 18.0}))
 
 
 @pytest.fixture(scope="module")
 def di():
-    import pandas as pd
-
-    load_reference()
-    from libreco.data import DatasetFeat, split_by_ratio_chrono
-
-    data = pd.read_csv(os.path.join(REFERENCE_ROOT, "examples/sample_data/sample_movielens_merged.csv"))
-    train, _ = split_by_ratio_chrono(data, test_size=0.2)
-    _, info = DatasetFeat.build_trainset(train, ["sex", "age", "occupation"], ["genre1", "genre2", "genre3"],
-                                         ["sex", "occupation", "genre1", "genre2", "genre3"], ["age"])
-    return info
+    return load_feat_data_info()
 
 
 def _spec(di):
@@ -48,9 +41,6 @@ def _spec(di):
 
 @pytest.mark.parametrize("name", ["FM", "DeepFM"])
 def test_single_user_feature_override_matches_reference_feed(di, name):
-    from libreco.prediction.preprocess import set_temp_feats
-    from libreco.recommendation.preprocess import _get_original_feats
-
     from librecommender_b200 import feat_models as fm
     from librecommender_b200.recommendation import recommend_tf_feat
     from oracle import ranking as orc
@@ -66,9 +56,9 @@ def test_single_user_feature_override_matches_reference_feed(di, name):
     model = types.SimpleNamespace(b200_engine=engine, n_items=di.n_items, n_users=di.n_users, task="ranking",
                                   data_info=di, user_consumed=di.user_consumed, model_name=name)
     N = di.n_items
-    for user, feats in ((5, {"sex": "F", "age": 40.0}), (11, {"occupation": 3}), (di.n_users, {"age": 18.0})):
-        sp, de = _get_original_feats(di, user, N, True, True)                    # the reference's own feed
-        sp, de = set_temp_feats(di, sp, de, feats)
+    ref_feed = load_reference_answers()
+    for c, (user, feats) in enumerate(override_cases(di.n_users)):
+        sp, de = ref_feed["feed_sparse"][c], ref_feed["feed_dense"][c]           # the reference's own feed
         preds = fwd(w, np.repeat(user, N), np.arange(N), sp.astype(np.int64), de.astype(np.float32),
                     dtype=np.float64).astype(np.float32)
         for n_rec in (7, 50):

@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 from oracle import ranking as orc
-from oracle.ref_loader import reference_available
+from _fixtures import load_reference_answers
 
 
 def _dict_from_csr(indptr, idx):
@@ -73,13 +73,7 @@ def test_embed_matches_reference_golden(path):
         assert (got == g[key]).mean() > 0.999
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference tree not present (GPU box)")
-def test_oracle_vs_live_reference_random():
-    from oracle.ref_loader import load_reference
-
-    load_reference()
-    from libreco.recommendation import rank_recommendations as ref_rank
-
+def random_rank_cases():
     rng = np.random.default_rng(5)
     for trial in range(20):
         B, N = int(rng.integers(1, 6)), int(rng.integers(5, 400))
@@ -88,10 +82,16 @@ def test_oracle_vs_live_reference_random():
         consumed = {u: rng.choice(N, size=int(rng.integers(0, N)), replace=False).tolist()
                     for u in range(B)}
         consumed = {u: v for u, v in consumed.items() if v}
-        uids = list(range(B))
-        ref = ref_rank("ranking", uids, preds, K, N, consumed, True, False, False)
+        yield list(range(B)), preds, K, N, consumed
+
+
+def test_oracle_vs_live_reference_random():
+    """Random shapes and consumed lists against the reference's rank_recommendations
+    (tests/golden/reference_answers.npz, tests/golden/gen_reference_answers.py)."""
+    g = load_reference_answers()
+    for trial, (uids, preds, K, N, consumed) in enumerate(random_rank_cases()):
         got = orc.rank_recommendations("ranking", uids, preds, K, N, consumed, True)
-        np.testing.assert_array_equal(ref, got)
+        np.testing.assert_array_equal(g[f"rank_{trial}"], got)
 
 
 def test_assign_oov_and_predict():

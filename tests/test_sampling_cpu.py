@@ -1,6 +1,6 @@
 """CPU: (1) the host parity samplers reproduce the reference's sampled indices BIT-EXACTLY under a
-fixed seed (golden vectors from the unmodified reference + live comparison when the reference tree
-is present); (2) the oracle's Philox restatement is self-consistent (known-answer vector)."""
+fixed seed (golden vectors from the unmodified reference, tests/golden/gen_sampling.py and
+tests/golden/gen_reference_answers.py); (2) the oracle's Philox restatement is self-consistent (known-answer vector)."""
 import os
 import random
 
@@ -8,7 +8,8 @@ import numpy as np
 import pytest
 
 from oracle import sampling as osm
-from oracle.ref_loader import reference_available
+
+from _fixtures import load_reference_answers
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "sampling.npz")
 
@@ -44,22 +45,22 @@ def test_parity_mode_bit_exact_against_reference_golden():
         osm.check_reference_invariants(got, g["users"], g["items_pos"], num_neg, n_items, consumed)
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference tree not present (GPU box)")
-def test_parity_mode_vs_live_reference():
-    from oracle.ref_loader import load_reference
-
-    load_reference()
-    from libreco.sampling import negatives as ref
-    from librecommender_b200 import sampling as S
-
+def random_negative_cases():
     gen = np.random.default_rng(9)
     for trial in range(5):
         n_items = int(gen.integers(20, 3000))
         pos = gen.integers(0, n_items, size=int(gen.integers(1, 500)))
         num_neg = int(gen.integers(1, 6))
-        a = ref.negatives_from_random(np.random.default_rng(trial), n_items, pos, num_neg)
+        yield n_items, pos, num_neg
+
+
+def test_parity_mode_vs_live_reference():
+    from librecommender_b200 import sampling as S
+
+    g = load_reference_answers()
+    for trial, (n_items, pos, num_neg) in enumerate(random_negative_cases()):
         b = S.negatives_from_random(np.random.default_rng(trial), n_items, pos, num_neg)
-        np.testing.assert_array_equal(a, b)
+        np.testing.assert_array_equal(g[f"negatives_{trial}"], b)
 
 
 def test_probs_from_frequency_and_philox_known_answer():

@@ -1,11 +1,12 @@
 """Round trips through the reference's on-disk weight formats (utils/save_load.py:39-98,
-bases/embed_base.py:289-330); with the reference mounted, its own loader reads our files."""
+bases/embed_base.py:289-330); the reference's own default_recs file (tests/golden/reference_default_recs.npz,
+written by tests/golden/gen_reference_answers.py) pins that format."""
 import os
 
 import numpy as np
 import pytest
 
-from oracle.ref_loader import load_reference, reference_available
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def test_embed_and_tf_variable_roundtrip(tmp_path):
@@ -36,15 +37,18 @@ def test_embed_and_tf_variable_roundtrip(tmp_path):
     np.testing.assert_array_equal(io.load_default_recs(str(tmp_path), "m"), np.arange(20))
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference not mounted")
 def test_reference_loader_reads_our_default_recs(tmp_path):
-    load_reference()
-    from libreco.utils.save_load import load_default_recs as ref_load
-
+    """Our file has the layout of the reference's (utils/save_load.py:39-48 reads key "default_recs" of
+    ``<name>_default_recs.npz``), and our loader reads the reference's file."""
     from librecommender_b200 import weights_io as io
 
     io.save_default_recs(str(tmp_path), "m", np.arange(2000))
-    np.testing.assert_array_equal(ref_load(str(tmp_path), "m"), np.arange(2000))
+    ours = np.load(os.path.join(tmp_path, "m_default_recs.npz"))
+    ref = np.load(os.path.join(GOLDEN, "reference_default_recs.npz"))
+    assert ours.files == ref.files
+    assert ours["default_recs"].dtype == ref["default_recs"].dtype
+    np.testing.assert_array_equal(ours["default_recs"], ref["default_recs"])
+    np.testing.assert_array_equal(io.load_default_recs(GOLDEN, "reference"), np.arange(2000))
 
 
 @pytest.mark.parametrize("arch,n_hidden,use_bn", [("FM", 0, True), ("DeepFM", 3, True), ("DeepFM", 2, False),
